@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — frames/sec of the MIMO denoising path on B200 (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]            our engine (one JSON line on rank 0)
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   our engine (one JSON line on rank 0)
   python bench.py --impl reference [--gpus N] --steps K --warmup W   the oracle port on the host cores
 
 Workload (BASELINE.json configs[1]): 512x512, 24 frames, 20 DDIM steps, CFG 3.5, fp16, synthetic PIL inputs,
@@ -129,6 +129,30 @@ class ClockSampler:
                 "power_w_max": max(pw) if pw else None, "samples": len(sm), "reasons": reasons}
 
 
+DUMP_BYTES = 60 << 20  # what --dump-outputs may write in all: under 64 MB with the .npy headers
+
+
+def dump_outputs(outputs: dict, dest: Path) -> None:
+    """Writes each output tensor as <dest>/<name>.npy in float32, DUMP_BYTES in all. An output larger than its share of
+    what is left is stored as a sample: its elements at the sorted flat indices that torch.randperm draws from a generator
+    seeded with 0. The sample depends only on the output's size, so runs with the same arguments store the same
+    elements."""
+    dest.mkdir(parents=True, exist_ok=True)
+    items = sorted(outputs.items(), key=lambda kv: kv[1].numel())
+    left = DUMP_BYTES
+    for i, (name, t) in enumerate(items):
+        flat = t.detach().float().cpu().reshape(-1)
+        share = left // (len(items) - i) // 4
+        if flat.numel() <= share:
+            arr, what = flat.reshape(t.shape).numpy(), "all"
+        else:
+            idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:share].sort().values
+            arr, what = flat[idx].numpy(), f"{share} seeded flat-index samples"
+        np.save(dest / f"{name}.npy", arr)
+        left -= arr.nbytes
+        print(f"bench.py: {dest / name}.npy <- {name} {tuple(t.shape)}: {what}", file=sys.stderr)
+
+
 def measured_peaks():
     p = ROOT / "MEASURED_PEAKS.json"
     if p.exists():
@@ -218,6 +242,8 @@ def run_ours(args):
     ms = e0.elapsed_time(e1)
     launches = ops.launches() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # after the clock sampler: the dump keeps the GPU idle for seconds
+        dump_outputs(out, Path(args.dump_outputs))
     pipe._collect_timings()
     phases = dict(pipe.timings)
     if world > 1:
@@ -235,7 +261,7 @@ def run_ours(args):
     res = warm.pop()
     del warm
     sync()
-    k_e2e = max(1, min(args.steps, 3))
+    k_e2e = args.steps
     t0 = time.perf_counter()
     for i in range(k_e2e):
         res = pipe(ref_img, poses, bks, WIDTH, HEIGHT, FRAMES, DDIM_STEPS, GUIDANCE, generator=clip_seed(i))
@@ -547,12 +573,18 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=2, help="BASELINE.json config number: 2 (default, the metric), 4, 5")
     ap.add_argument("--dump-calls", default=None, help="write every profiled C-ABI call (name, flops, bytes, ms) as CSV")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step returned (latents, videos) as DIR/<name>.npy, float32")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU sample (development runs)")
     ap.add_argument("--no-breakdown", action="store_true",
                     help="skip the two extra diagnostic clips (event-bracketed calls, CUPTI table): roofline = null")
     ap.add_argument("--one-clip", action="store_true",
                     help="run exactly one device-resident clip and exit (for `ncu` launch lists; not a bench value)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.one_clip or args.impl == "reference"):
+        ap.error("--dump-outputs writes the timed steps of our engine: not with --one-clip or --impl reference")
     select_config(args.config)
     if args.impl == "reference":
         run_reference(args)

@@ -97,3 +97,20 @@ def test_usable_cores_and_extrapolation(bench_mod):
     assert 1 <= b.usable_cores() <= 4096
     fx = {"t_ref": 1.0, "t_dec": 2.0, "t_enc": 3.0}
     assert b._extrapolate(10.0, 8, fx) == 20 * 10.0 * 3 + 24 * 2.0 + 2 * 3.0 + 1.0
+
+
+def test_dump_outputs_budget_and_sample(bench_mod, tmp_path):
+    """--dump-outputs: small outputs whole, a large one as a fixed seeded sample; float32, DUMP_BYTES in all."""
+    import torch
+    b = bench_mod
+    lat = torch.randn(1, 4, 24, 64, 64, dtype=torch.float16)
+    vid = torch.rand(1, 3, 24, 512, 512, dtype=torch.float16)
+    for d in ("a", "b"):
+        b.dump_outputs({"latents": lat, "videos": vid}, tmp_path / d)
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("latents", "videos")}
+    assert got["latents"].dtype == got["videos"].dtype == np.float32
+    assert np.array_equal(got["latents"], lat.float().numpy())
+    assert got["videos"].ndim == 1 and 0 < got["videos"].size < vid.numel()
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) < 64 * 1000 * 1000
+    assert np.array_equal(got["videos"], np.load(tmp_path / "b" / "videos.npy"))
+    assert np.isin(got["videos"], vid.float().numpy().reshape(-1)).all()

@@ -1,24 +1,27 @@
-"""Drop-in boundary proof (SURVEY.md §8b) with the reference's own, UNMODIFIED files, on CPU:
+"""Drop-in boundary proof (SURVEY.md §8b) against the reference's own, UNMODIFIED files, on CPU. The reference is not
+part of this repository: oracle/gen_dropin_golden.py runs its files over this repo's module facades and stores what they
+did under tests/golden/; the tests below hold this repo's code to those recordings. There is no GPU here and the product
+has no CPU path, so the facades' engines are replaced - in these tests only - by oracle-backed stand-ins
+(oracle/dropin.py).
 
-1. `src/pipelines/pipeline_pose2vid_long_edit_bkfill_roiclip.py` is loaded verbatim from /root/reference; its
-   `from src.models... / src.pipelines...` imports resolve to THIS repo's overlay (`src/`), `diffusers` to the oracle's
-   compat package. Its Pose2VideoPipeline is constructed over this repo's module facades and scheduler and run for
-   BASELINE config 1. There is no GPU here and the product has no CPU path, so the facades' engines are replaced — in
-   this test only — by oracle-backed stand-ins; everything between the pipeline file and the engine entry points (call
-   signatures, reference tensor layouts, CFG ordering, the ReferenceAttentionControl handshake, DDIMScheduler.step) is
-   the shipped host code. The result must equal the golden clip the reference's pipeline produced over the reference's
-   own modules (tests/golden/pipeline_cfg1.pt).
-2. run_animate.py's model-construction block (MIMO.__init__, :60-129) is executed statement by statement from the
-   reference file over the facades (`AutoencoderKL.from_pretrained`, `UNet2DConditionModel.from_pretrained`,
-   `UNet3DConditionModel.from_pretrained_2d`, `PoseGuider(...)`, `DDIMScheduler(**kwargs)`, `load_state_dict`,
-   `Pose2VideoPipeline(...).to(...)`) against throw-away checkpoints; the only edit is the device literal
-   "cuda" -> "cpu". The reference's configs/inference/inference_v2.yaml is read as it is.
-
-The reference tree exists only in the build container: skipped elsewhere (the GPU box)."""
-import ast
-import importlib.util
+1. `src/pipelines/pipeline_pose2vid_long_edit_bkfill_roiclip.py`, loaded verbatim with its `src.*` imports resolved to
+   THIS repo's overlay (`src/`), ran its Pose2VideoPipeline over the module facades and scheduler for BASELINE config 1
+   and a 26-frame two-window clip. Every call it made on them - `UNet3DConditionModel(sample, t,
+   encoder_hidden_states=..., pose_cond_fea=..., return_dict=False)[0]`, `PoseGuider(...)`, `AutoencoderKL.encode(...)
+   .latent_dist.mean` / `.decode(...).sample`, `UNet2DConditionModel(...)`, `ReferenceAttentionControl(...)`, `.update`,
+   `.clear`, `DDIMScheduler.set_timesteps / scale_model_input / step(...).prev_sample` - is in
+   tests/golden/dropin_facade_trace.*; the calls are replayed here through the facades and must return what they
+   returned. The clips it produced (tests/golden/dropin_pipeline.pt) must also come out of this repo's own sampler.
+2. run_animate.py's model-construction block (MIMO.__init__, :60-129), executed statement by statement over the facades
+   against throw-away checkpoints (the only edit: the device literal "cuda" -> "cpu"), made the calls recorded in
+   tests/golden/run_animate_init_trace.json (`AutoencoderKL.from_pretrained`, `UNet2DConditionModel.from_pretrained`,
+   `UNet3DConditionModel.from_pretrained_2d` with the reference's configs/inference/inference_v2.yaml values,
+   `PoseGuider(...)`, `DDIMScheduler(**kwargs)`, `load_state_dict`, `Pose2VideoPipeline(...).to(...)`). They are
+   replayed here, in order, and must build the same pipeline.
+3. run_edit.py's scene-compositing loop and src/pipelines/utils.py: their outputs on seeded inputs."""
+import hashlib
+import importlib
 import json
-import sys
 from pathlib import Path
 from types import SimpleNamespace
 
@@ -26,257 +29,139 @@ import numpy as np
 import pytest
 import torch
 
-ROOT = Path(__file__).resolve().parents[1]
-REF = Path("/root/reference")
-pytestmark = pytest.mark.skipif(not (REF / "src" / "pipelines").exists(), reason="reference tree not present")
-
-PIPE_FILE = REF / "src" / "pipelines" / "pipeline_pose2vid_long_edit_bkfill_roiclip.py"
+from oracle.dropin import (TRACE_CASES, composite_case, follow, load_trace, make_checkpoints, oracle_engines, out_sample,
+                           resolve, trace_case)
 
 
-@pytest.fixture()
-def compat_path():
-    added = [str(ROOT / "oracle" / "diffusers_shim"), str(ROOT / "tests" / "compat")]
-    for p in added:
-        sys.path.insert(0, p)
-    yield
-    for p in added:
-        sys.path.remove(p)
-
-
-def _load_reference_pipeline():
-    spec = importlib.util.spec_from_file_location("_reference_pipeline_file", PIPE_FILE)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
-
-
-def _oracle_engines(monkeypatch, O, cfg, vcfg):
-    """Stand-ins for the four engine factories, backed by the oracle (fp32, CPU)."""
-    from mimo_b200 import ops
+@pytest.mark.parametrize("F_,size", TRACE_CASES)
+def test_reference_pipeline_facade_calls_replay(monkeypatch, golden_dir, F_, size):
+    """Every facade call the reference's pipeline file made, in its order, with its arguments (large ones rebuilt from
+    what the replay computed before), through the facades: each must return the same structure, shape and values."""
     from mimo_b200.host import modules as M
+    from oracle import torch_oracle as O
+    rec, arrays = load_trace(golden_dir, F_)
+    c = trace_case(F_, size)
+    oracle_engines(monkeypatch, O, c.cfg, c.vcfg)
+    objs, pool, made = dict(c.models), {}, set()
 
-    def ncfhw_to_nhwc(src, cpad, dtype, out=None):
-        b, c, f, h, w = src.shape
-        t = src.permute(0, 2, 3, 4, 1).reshape(b * f * h * w, c).to(dtype)
-        return torch.nn.functional.pad(t, (0, cpad - c))
+    def dec(v):
+        if isinstance(v, list):
+            return [dec(x) for x in v]
+        if not isinstance(v, dict):
+            return v
+        if "tensor" in v:
+            return resolve(v["tensor"], pool, arrays)
+        if "obj" in v:
+            return objs[v["obj"]]
+        if "device" in v:
+            return torch.device(v["device"])
+        return torch.Generator()
 
-    def nhwc_to_ncfhw(src, b, c, f, h, w, out_dtype=None, out=None):
-        return src[:, :c].reshape(b, f, h, w, c).permute(0, 4, 1, 2, 3).contiguous()
-
-    monkeypatch.setattr(ops, "ncfhw_to_nhwc", ncfhw_to_nhwc)
-    monkeypatch.setattr(ops, "nhwc_to_ncfhw", nhwc_to_ncfhw)
-    monkeypatch.setattr(M._EngineModel, "_require_cuda", lambda self: None)
-
-    class Den:
-        def __init__(self, sd):
-            self.sd, self.clip_state = sd, None
-
-        def begin_clip(self, ehs, banks, cfg, frames, branches=None):
-            self.clip_state = {"ehs": ehs, "banks": banks, "cfg": cfg}
-
-        def set_cross_attn(self, ehs):
-            self.clip_state["ehs"] = ehs
-
-        def forward(self, sample, timestep, pose_nhwc):
-            b, c, f, h, w = sample.shape
-            pose = pose_nhwc.reshape(b, f, h, w, -1).permute(0, 4, 1, 2, 3)
-            st = self.clip_state
-            # the host layer hands over the conditional half of the banks only (the unconditional half is never read);
-            # the oracle restates the reference, which keeps both: fill the unused slot with a copy
-            banks = {k: (v if v.shape[0] == b else v.repeat(b, 1, 1)) for k, v in st["banks"].items()}
-            return O.denoising_unet(self.sd, sample, int(timestep), st["ehs"], pose, banks, cfg, cfg=st["cfg"])
-
-    class Ref:
-        def __init__(self, sd):
-            self.sd = sd
-
-        def write_banks(self, latents, ehs, reader):
-            return O.reference_unet_banks(self.sd, latents, ehs, cfg)
-
-    class Pose:
-        def __init__(self, sd):
-            self.sd = sd
-
-        def forward(self, cond):
-            y = O.pose_guider(self.sd, cond)  # [b, C, F, h, w]
-            return y.permute(0, 2, 3, 4, 1).reshape(-1, y.shape[1])
-
-    class Vae:
-        def __init__(self, sd):
-            self.sd = sd
-
-        def encode_mean(self, x):
-            return O.vae_encode_mean(self.sd, x, vcfg)
-
-        def decode(self, z):
-            return O.vae_decode(self.sd, z, vcfg)
-
-    def cached(factory):
-        def engine(self):
-            if self._engine is None:
-                self._engine = factory(self.state_dict())
-            return self._engine
-        return engine
-
-    monkeypatch.setattr(M.UNet3DConditionModel, "engine", cached(Den))
-    monkeypatch.setattr(M.UNet2DConditionModel, "engine", cached(Ref))
-    monkeypatch.setattr(M.PoseGuider, "engine", cached(Pose))
-    monkeypatch.setattr(M.AutoencoderKL, "engine", cached(lambda sd: (Vae(sd), Vae(sd))))
+    with torch.no_grad():
+        for k, e in enumerate(rec["calls"]):
+            if "extra" in e:  # the initial noise
+                pool[f"o{k}"] = resolve(e["extra"], pool, arrays)
+                continue
+            args, kwargs = dec(e["args"]), {n: dec(v) for n, v in e["kwargs"].items()}
+            if e["method"] is None:
+                out = objs[f"rac{k}"] = M.ReferenceAttentionControl(*args, **kwargs)
+            else:
+                out = getattr(objs[e["obj"]], e["method"])(*args, **kwargs)
+            made.add((e["obj"], e["method"]))
+            if "out" not in e:
+                continue
+            got = follow(out, e["out"]["path"])
+            assert list(got.shape) == e["out"]["shape"], (k, e["obj"], e["method"])
+            s, want = torch.from_numpy(out_sample(got).numpy()), torch.from_numpy(arrays[f"s{k}"])
+            assert float((s - want).norm()) <= 1e-4 * float(want.norm()) + 1e-6, (k, e["obj"], e["method"], s, want)
+            pool[f"o{k}"] = got
+    assert {("den", "__call__"), ("refu", "__call__"), ("pg", "__call__"), ("vae", "encode"), ("vae", "decode"),
+            ("sched", "step"), ("sched", "scale_model_input"), ("sched", "set_timesteps")} <= made
+    assert {m for o, m in made if o.startswith("rac")} == {"update", "clear"}
+    assert c.models["den"]._engine.clip_state is None  # reference_control_reader.clear() reached the engine
 
 
 @pytest.mark.parametrize("F_,guidance", [(1, 3.5), (26, 3.5), (26, 1.0)])
-def test_reference_pipeline_file_runs_over_the_facades(compat_path, monkeypatch, golden_dir, F_, guidance):
-    import PIL.Image
-    from transformers import CLIPVisionConfig, CLIPVisionModelWithProjection
+def test_reference_pipeline_file_runs_over_the_facades(monkeypatch, golden_dir, F_, guidance):
+    """The clip (sampled every `stride` pixels), its mean and the callbacks the reference's pipeline file produced over
+    the facades (tests/golden/dropin_pipeline.pt), against this repo's sampler on the same models and inputs and against
+    the oracle. The facade calls of that run are replayed by test_reference_pipeline_facade_calls_replay."""
+    from test_pipeline_plumbing_cpu import own_sampler_clip
 
-    from mimo_b200.host import modules as M
-    from mimo_b200.host.scheduler import DDIMScheduler
-    from oracle import torch_oracle as O
-    ref_mod = _load_reference_pipeline()
-    # the pipeline file's intra-package imports landed on this repo's overlay
-    assert ref_mod.ReferenceAttentionControl is M.ReferenceAttentionControl
     from mimo_b200.host import context
-    assert ref_mod.get_context_scheduler is context.get_context_scheduler
-
-    g = torch.load(golden_dir / "pipeline_cfg1.pt")
-    seed, size, steps = g["seed"], g["size"], g["steps"]
-    assert g["F"] == 1
-    vae_widths = tuple(g["vae_widths"])
-    if F_ != 1:  # two context windows (24 + wrap-around): checked against oracle.sample_clip instead of the fixture
-        seed, size, vae_widths = 300, 64, (32, 64, 128, 128)
-    widths = (128, 256, 512, 512)
-    cfg, vcfg = O.UNetConfig(block_out_channels=widths), O.VAEConfig(block_out_channels=vae_widths)
-    _oracle_engines(monkeypatch, O, cfg, vcfg)
-    mk = dict(num_attention_heads=8, num_transformer_block=1, attention_block_types=["Temporal_Self", "Temporal_Self"],
-              temporal_position_encoding=True, temporal_position_encoding_max_len=32, temporal_attention_dim_div=1)
-    den = M.UNet3DConditionModel(block_out_channels=widths, cross_attention_dim=768, use_inflated_groupnorm=True,
-                                 use_motion_module=True, motion_module_mid_block=True, motion_module_type="Vanilla",
-                                 motion_module_kwargs=mk, unet_use_cross_frame_attention=False,
-                                 unet_use_temporal_attention=False)
-    ref = M.UNet2DConditionModel(block_out_channels=widths, cross_attention_dim=768)
-    pg = M.PoseGuider(widths[0], conditioning_channels=3, block_out_channels=(16, 32, 96, 256))
-    vae = M.AutoencoderKL(block_out_channels=vae_widths)
-    sds = dict(den=O.make_denoising_unet_sd(cfg, seed), ref=O.make_reference_unet_sd(cfg, seed + 1),
-               pg=O.make_pose_guider_sd(seed + 2, widths[0]), vae=O.make_vae_sd(vcfg, seed + 3))
-    for m, k in ((den, "den"), (ref, "ref"), (pg, "pg"), (vae, "vae")):
-        m.load_state_dict(sds[k], strict=True)
-    torch.manual_seed(seed + 4)
-    clip = CLIPVisionModelWithProjection(CLIPVisionConfig(hidden_size=64, intermediate_size=128, num_hidden_layers=2,
-                                                          num_attention_heads=4, image_size=224, patch_size=32,
-                                                          projection_dim=cfg.cross_attention_dim)).eval()
-    sched = DDIMScheduler(beta_start=0.00085, beta_end=0.012, beta_schedule="scaled_linear", clip_sample=False,
-                          steps_offset=1, prediction_type="v_prediction", rescale_betas_zero_snr=True,
-                          timestep_spacing="trailing")
-    pipe = ref_mod.Pose2VideoPipeline(vae=vae, image_encoder=clip, reference_unet=ref, denoising_unet=den,
-                                      pose_guider=pg, scheduler=sched)
-    rng = np.random.RandomState(seed)
-    ref_img = PIL.Image.fromarray(rng.randint(0, 256, (size, size, 3), dtype=np.uint8))
-    poses, bks = [], []
-    for i in range(F_):
-        a = np.zeros((size, size, 3), np.uint8)
-        a[size // 4: size // 2 + i % 8, size // 3: size // 3 + 40] = rng.randint(11, 256, 3)
-        poses.append(PIL.Image.fromarray(a))
-        bks.append(PIL.Image.fromarray(rng.randint(0, 256, (size, size, 3), dtype=np.uint8)))
-    seen = []
-    with torch.no_grad():
-        out = pipe(ref_img, poses, bks, size, size, F_, steps, guidance, generator=torch.manual_seed(42),
-                   callback=lambda i, t, lat: seen.append((i, int(t))), callback_steps=1)
+    from mimo_b200.host import modules as M
+    want = torch.load(golden_dir / "dropin_pipeline.pt")
+    # the pipeline file's intra-package imports land on this repo's overlay
+    for mod, names in want["imports"]:
+        for n in names:
+            assert hasattr(importlib.import_module(mod), n), (mod, n)
+    assert importlib.import_module("src.models.mutual_self_attention").ReferenceAttentionControl is M.ReferenceAttentionControl
+    assert importlib.import_module("src.pipelines.context").get_context_scheduler is context.get_context_scheduler
+    w = want["cases"][f"{F_}-{guidance}"]
+    r = own_sampler_clip(monkeypatch, golden_dir, F_, guidance)
     # the callback sees the inner loop's shadowed variable (:503-510): the index of the last context batch, at every step
-    assert seen == [(0 if F_ == 1 else 1, 999), (0 if F_ == 1 else 1, 499)]
-    vid = out.videos
-    assert vid.shape == (1, 3, F_, size, size) and vid.dtype == torch.float32
+    assert [(i, t) for i, t, _ in r.seen] == w["seen"] == [(0 if F_ == 1 else 1, 999), (0 if F_ == 1 else 1, 499)]
+    assert len(r.never) == w["never"]  # callback_steps = 2: called only where the last batch index is even
+    s, gv = w["stride"], w["videos"]
+    vid = r.out["videos"].float()
+    assert vid.shape == tuple(w["shape"])
+    err = float((vid[:, :, :, ::s, ::s] - gv).norm() / gv.norm())
+    assert err < 1e-4, err  # fp32 both sides
+    assert abs(float(vid.mean()) - w["videos_mean"]) < 1e-5
     if F_ == 1:
-        want = g["videos"].float()
-        got = vid[:, :, :, ::8, ::8]
-        err = float((got - want).norm() / want.norm())
-        assert err < 2e-3, err  # the fixture is stored in fp16
-        assert abs(float(vid.mean()) - g["videos_mean"]) < 1e-4
+        g = torch.load(golden_dir / "pipeline_cfg1.pt")  # the same clip from the reference's own modules
+        gc = g["videos"].float()[:, :, :, ::s // 8, ::s // 8]  # stored every 8 pixels
+        assert float((gv - gc).norm() / gc.norm()) < 2e-3  # stored in fp16
+        assert abs(w["videos_mean"] - g["videos_mean"]) < 1e-4
     else:
-        from mimo_b200.host.pipeline import pil_to_tensor
-        never = []
-        with torch.no_grad():
-            pipe(ref_img, poses, bks, size, size, F_, 1, guidance, generator=torch.manual_seed(42),
-                 callback=lambda *a: never.append(a), callback_steps=2)
-            assert never == []  # 1 % 2 != 0: with two windows and callback_steps = 2 the reference never calls back
-            emb = clip(pipe.clip_image_processor.preprocess(ref_img.resize((224, 224)), return_tensors="pt").pixel_values).image_embeds
-            lat0 = torch.randn((1, 4, F_, size // 8, size // 8), generator=torch.manual_seed(42), dtype=torch.float32)
-            W = O.Weights(sds["den"], sds["ref"], sds["pg"], sds["vae"], cfg, vcfg)
-            ref_out = O.sample_clip(W, pil_to_tensor(ref_img, size, size, True),
-                                    pil_to_tensor(poses, size, size, False).permute(1, 0, 2, 3).unsqueeze(0),
-                                    pil_to_tensor(bks, size, size, True), emb, lat0, steps, guidance)
-        err = float((vid - ref_out["videos"]).norm() / ref_out["videos"].norm())
-        assert err < 1e-4, err  # fp32 both sides
-    assert den._engine.clip_state is None  # reference_control_reader.clear() reached the engine
+        want_o = r.ref_out["videos"][:, :, :, ::s, ::s]
+        err = float((gv - want_o).norm() / want_o.norm())
+        assert err < 1e-4, err
+    assert r.den._engine.clip_state is None  # reference_control_reader.clear() reached the engine
 
 
-def _make_checkpoints(tmp: Path):
-    """Throw-away 'pretrained_weights' in the directory layout run_animate.py reads (tiny widths: files stay small)."""
-    from safetensors.torch import save_file
-    from transformers import CLIPVisionConfig, CLIPVisionModelWithProjection
+def _replay(trace, names, tmp: Path):
+    """Makes the recorded calls in order: `target` is a name in `names` or "$k", the result of call k."""
+    got = []
 
-    from mimo_b200.host import schema
-    widths = (32, 64, 64, 64)
-    gen = torch.Generator().manual_seed(0)
-    rnd = lambda shapes: {k: torch.randn(s, generator=gen) * 0.02 for k, s in shapes.items()}
-    base = tmp / "stable-diffusion-v1-5" / "unet"
-    base.mkdir(parents=True)
-    (base / "config.json").write_text(json.dumps(dict(
-        sample_size=64, in_channels=4, out_channels=4, block_out_channels=list(widths), layers_per_block=2,
-        cross_attention_dim=768, attention_head_dim=8, norm_num_groups=32, norm_eps=1e-5)))
-    sd15 = rnd(schema.unet_schema(widths, 2, 768, in_channels=4, out_channels=4, motion=False, out_head=True))
-    save_file(sd15, str(base / "diffusion_pytorch_model.safetensors"))
-    den_full = rnd(schema.unet_schema(widths, 2, 768, in_channels=8, out_channels=4, motion=True, out_head=True))
-    torch.save({k: v for k, v in den_full.items() if "motion_modules" in k}, tmp / "motion_module.pth")
-    torch.save(den_full, tmp / "denoising_unet.pth")
-    torch.save({k: v for k, v in sd15.items() if not k.startswith(("conv_norm_out", "conv_out"))}, tmp / "reference_unet.pth")
-    torch.save(rnd(schema.pose_guider_schema(320, 3, (16, 32, 96, 256))), tmp / "pose_guider.pth")
-    vae = tmp / "sd-vae-ft-mse"
-    vae.mkdir()
-    vw = (32, 32, 64, 64)
-    (vae / "config.json").write_text(json.dumps(dict(block_out_channels=list(vw), layers_per_block=2, latent_channels=4,
-                                                     in_channels=3, out_channels=3, norm_num_groups=32,
-                                                     scaling_factor=0.18215)))
-    save_file(rnd(schema.vae_schema(vw, 2, 4, 3, 3)), str(vae / "diffusion_pytorch_model.safetensors"))
-    CLIPVisionModelWithProjection(CLIPVisionConfig(hidden_size=32, intermediate_size=64, num_hidden_layers=1,
-                                                   num_attention_heads=2, image_size=224, patch_size=32,
-                                                   projection_dim=768)).save_pretrained(tmp / "image_encoder")
-    cfg = tmp / "animation_edit.yaml"
-    cfg.write_text("\n".join([
-        f'pretrained_base_model_path: "{tmp / "stable-diffusion-v1-5"}"', f'pretrained_vae_path: "{vae}"',
-        f'image_encoder_path: "{tmp / "image_encoder"}"', f'denoising_unet_path: "{tmp / "denoising_unet.pth"}"',
-        f'reference_unet_path: "{tmp / "reference_unet.pth"}"', f'pose_guider_path: "{tmp / "pose_guider.pth"}"',
-        f'motion_module_path: "{tmp / "motion_module.pth"}"',
-        f'inference_config: "{REF / "configs" / "inference" / "inference_v2.yaml"}"', "weight_dtype: 'fp16'"]))
-    return cfg
+    def dec(v):
+        if isinstance(v, list):
+            return [dec(x) for x in v]
+        if not isinstance(v, dict):
+            return v
+        if "ref" in v:
+            return got[v["ref"]]
+        if "path" in v:
+            return str(tmp / v["path"])
+        if "dtype" in v:
+            return getattr(torch, v["dtype"])
+        if "tuple" in v:
+            return tuple(dec(v["tuple"]))
+        return {k: dec(x) for k, x in v["dict"].items()}
+
+    for e in trace:
+        t = e["target"]
+        obj = got[int(t[1:])] if t.startswith("$") else names[t]
+        fn = obj if e["attr"] is None else getattr(obj, e["attr"])
+        got.append(fn(*dec(e["args"]), **{k: dec(x) for k, x in e["kwargs"].items()}))
+    return got
 
 
-class _CudaToCpu(ast.NodeTransformer):
-    def visit_Constant(self, node):
-        return ast.copy_location(ast.Constant("cpu"), node) if node.value == "cuda" else node
-
-
-def test_run_animate_model_construction_block(compat_path, tmp_path):
-    from omegaconf import OmegaConf
+def test_run_animate_model_construction_block(tmp_path, golden_dir):
     from transformers import CLIPVisionModelWithProjection
 
     from mimo_b200.host import modules as M
     from mimo_b200.host.pipeline import Pose2VideoPipeline
     from mimo_b200.host.scheduler import DDIMScheduler
-    cfg_file = _make_checkpoints(tmp_path)
-    tree = ast.parse((REF / "run_animate.py").read_text())
-    init = next(f for c in tree.body if isinstance(c, ast.ClassDef) and c.name == "MIMO"
-                for f in c.body if isinstance(f, ast.FunctionDef) and f.name == "__init__")
-    body = ast.Module(body=[_CudaToCpu().visit(st) for st in init.body], type_ignores=[])
-    ast.fix_missing_locations(body)
-    args = SimpleNamespace(config=str(cfg_file), W=512, H=512, seed=42, assets_dir=str(tmp_path))
-    import os
-    ns = dict(torch=torch, os=os, OmegaConf=OmegaConf, AutoencoderKL=M.AutoencoderKL, DDIMScheduler=DDIMScheduler,
-              UNet2DConditionModel=M.UNet2DConditionModel, UNet3DConditionModel=M.UNet3DConditionModel,
-              PoseGuider=M.PoseGuider, CLIPVisionModelWithProjection=CLIPVisionModelWithProjection,
-              Pose2VideoPipeline=Pose2VideoPipeline, parse_args=lambda: args, load_mask_list=lambda p: [],
-              self=SimpleNamespace(), debug_mode=False)
-    exec(compile(body, "run_animate.py:MIMO.__init__", "exec"), ns)
-    me = ns["self"]
+    make_checkpoints(tmp_path)
+    rec = json.loads((golden_dir / "run_animate_init_trace.json").read_text())
+    names = {"AutoencoderKL": M.AutoencoderKL, "DDIMScheduler": DDIMScheduler, "PoseGuider": M.PoseGuider,
+             "UNet2DConditionModel": M.UNet2DConditionModel, "UNet3DConditionModel": M.UNet3DConditionModel,
+             "CLIPVisionModelWithProjection": CLIPVisionModelWithProjection, "Pose2VideoPipeline": Pose2VideoPipeline,
+             "torch.load": torch.load}
+    assert {e["target"] for e in rec["calls"] if not e["target"].startswith("$")} <= set(names)
+    got = _replay(rec["calls"], names, tmp_path)
+    me = SimpleNamespace(pipe=got[rec["self"]["pipe"]["ref"]], width=rec["self"]["width"], height=rec["self"]["height"])
     pipe = me.pipe
     assert isinstance(pipe, Pose2VideoPipeline) and (me.width, me.height) == (512, 512)
     assert pipe.denoising_unet.dtype == torch.float16 and pipe.reference_unet.dtype == torch.float16
@@ -285,98 +170,56 @@ def test_run_animate_model_construction_block(compat_path, tmp_path):
     want = torch.load(tmp_path / "denoising_unet.pth")["conv_in.weight"].half()
     assert torch.equal(pipe.denoising_unet.state_dict()["conv_in.weight"], want)
     assert "down_blocks.0.motion_modules.0.temporal_transformer.proj_in.weight" in pipe.denoising_unet.state_dict()
-    # no GPU here: the first forward must fail loudly, never fall back to a CPU path
+    # the models must be the pipeline's: the construction block never rebinds them
+    assert pipe.pose_guider is got[next(i for i, e in enumerate(rec["calls"]) if e["target"] == "PoseGuider")]
+    # on the CPU the first forward must fail loudly, never fall back to a CPU path
     from mimo_b200.lib import MimoError
     with pytest.raises(MimoError):
         pipe.pose_guider(torch.zeros(1, 3, 1, 64, 64, dtype=torch.float16))
 
 
-def test_scene_compositing_matches_the_reference_loop(compat_path, monkeypatch):
-    """run_edit.py's post-processing loop (:253-304), executed from the reference file with tools/util.py's own get_mask,
-    against mimo_b200.host.composite.composite_clip on the same synthetic clip. The blend kernel needs a GPU, so here (and
-    only here) ops.composite_frame is the numpy oracle: this pins the helper's host logic (PIL resize / crop / paste,
-    INTER_AREA mask resize, mask placement, cross-fade factor, 16-way mask choice) AND the oracle's arithmetic to the
-    reference's code; the kernel is pinned to the oracle bit for bit on the GPU (tests/test_clip_composite_gpu.py)."""
-    import cv2
-    from PIL import Image
-
+def test_scene_compositing_matches_the_reference_loop(monkeypatch, golden_dir):
+    """run_edit.py's post-processing loop (:253-304) with tools/util.py's own get_mask composited composite_case(), with
+    and without an occlusion mask (tests/golden/run_edit_composite.json: SHA-256 and sum of every frame); here
+    mimo_b200.host.composite.composite_clip runs on the same clip. The blend kernel needs a GPU, so here (and only here)
+    ops.composite_frame is the numpy oracle: this pins the helper's host logic (PIL resize / crop / paste, INTER_AREA
+    mask resize, mask placement, cross-fade factor, 16-way mask choice) AND the oracle's arithmetic to the reference's
+    code; the kernel is pinned to the oracle bit for bit on the GPU (tests/test_clip_composite_gpu.py)."""
     from mimo_b200 import ops
     from mimo_b200.host import composite
     from oracle.composite_oracle import composite_frame
-    spec = importlib.util.spec_from_file_location("_reference_tools_util", REF / "tools" / "util.py")
-    ref_util = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref_util)
+    c = composite_case()
+    want = json.loads((golden_dir / "run_edit_composite.json").read_text())
 
-    rng = np.random.RandomState(3)
-    W, H, n_frames, overlay = 96, 72, 7, 2
-    contexts = [[0, 1, 2, 3, 4], [3, 4, 5, 6]]  # frames 3, 4 are composited twice: cross-fade
-    bboxes = [(0, 60, 4, 72), (20, 96, 0, 50)]   # touch different borders: different feather masks
-    bk = [Image.fromarray(rng.randint(0, 256, (H, W, 3), dtype=np.uint8)) for _ in range(n_frames)]
-    vid = [Image.fromarray(rng.randint(0, 256, (H, W, 3), dtype=np.uint8)) for _ in range(n_frames)]
-    occ = [Image.fromarray(np.repeat(rng.randint(0, 256, (H, W, 1), dtype=np.uint8), 3, axis=2)) for _ in range(n_frames)]
-    mask_list = [rng.rand(64, 64).astype(np.float32) for _ in range(16)]
-    pads, padvs = [], []
-    for k, ctx in enumerate(contexts):
-        w_min, w_max, h_min, h_max = bboxes[k]
-        bw, bh = w_max - w_min, h_max - h_min
-        side = max(bw, bh)
-        side += (16 - side % 16) % 16
-        top = (side - bh) // 2
-        left = (side - bw) // 2
-        for _ in ctx:
-            pads.append([side, side])
-            padvs.append([top, side - bh - top, left, side - bw - left])
-    video = torch.rand(3, sum(len(c) for c in contexts), 64, 64)
-
-    # ---- the reference's loop, verbatim from run_edit.py ----
-    tree = ast.parse((REF / "run_edit.py").read_text())
-    run = next(f for c in tree.body if isinstance(c, ast.ClassDef) and c.name == "MIMO"
-               for f in c.body if isinstance(f, ast.FunctionDef) and f.name == "run")
-    loop = next(st for st in run.body if isinstance(st, ast.For) and isinstance(st.iter, ast.Call)
-                and getattr(st.iter.func, "id", "") == "enumerate" and getattr(st.iter.args[0], "id", "") == "context_list")
-    init = next(st for st in run.body if isinstance(st, ast.Assign) and getattr(st.targets[0], "id", "") == "res_images")
-    idx0 = next(st for st in run.body if isinstance(st, ast.Assign) and getattr(st.targets[0], "id", "") == "video_idx")
-    mod = ast.Module(body=[idx0, init, loop], type_ignores=[])
-    ast.fix_missing_locations(mod)
-    me = SimpleNamespace(args=SimpleNamespace(L=n_frames), mask_list=mask_list)
-    ns = dict(np=np, cv2=cv2, Image=Image, get_mask=ref_util.get_mask, self=me, context_list=contexts,
-              bbox_clip_list=bboxes, bk_images_ori=bk, vid_images_ori=vid, occ_mask_images=occ,
-              clip_pad_list_context=pads, clip_padv_list_context=padvs, video=video, overlay=overlay)
-    exec(compile(mod, "run_edit.py:MIMO.run[post-process]", "exec"), ns)
-    want = ns["res_images"]
-
-    # ---- this repo's helper, with the blend evaluated by the oracle instead of the kernel ----
     def blend_on_cpu(canvas, bkf, mask, *, occ=None, vid=None, prev=None, factor=0.0, out=None):
         f = lambda t: None if t is None else t.cpu().numpy()
         return torch.from_numpy(composite_frame(f(canvas), f(bkf), f(mask), f(occ), f(vid), f(prev), factor))
 
     monkeypatch.setattr(ops, "composite_frame", blend_on_cpu)
-    got = composite.composite_clip(video, contexts, bboxes, bk, vid, occ, pads, padvs, mask_list, n_frames, overlay, device="cpu")
-    for i in range(n_frames):
-        assert want[i] is not None and got[i] is not None
-        assert np.array_equal(want[i], got[i]), (i, int((want[i].astype(int) - got[i].astype(int)).__abs__().max()))
-    # and without an occlusion mask (animate-style templates, run_edit.py:262-265)
-    ns.update(occ_mask_images=None)
-    exec(compile(mod, "run_edit.py:MIMO.run[post-process]", "exec"), ns)
-    got = composite.composite_clip(video, contexts, bboxes, bk, vid, None, pads, padvs, mask_list, n_frames, overlay, device="cpu")
-    for i in range(n_frames):
-        assert np.array_equal(ns["res_images"][i], got[i]), i
+    for key, occ in (("occ", c.occ), ("no_occ", None)):  # without: animate-style templates, run_edit.py:262-265
+        got = composite.composite_clip(c.video, c.contexts, c.bboxes, c.bk, c.vid, occ, c.pads, c.padvs, c.mask_list,
+                                       c.n_frames, c.overlay, device="cpu")
+        assert len(want[key]) == c.n_frames
+        for i, w in enumerate(want[key]):
+            f = np.ascontiguousarray(got[i], dtype=np.uint8)
+            assert list(f.shape) == w["shape"] and hashlib.sha256(f.tobytes()).hexdigest() == w["sha256"], (
+                key, i, int(f.sum(dtype=np.int64)) - w["sum"])
 
 
-def test_overlay_pipeline_utils_equal_the_reference():
+def test_overlay_pipeline_utils_equal_the_reference(golden_dir):
     """src/pipelines/utils.py (imported by the reference's pipeline file, dead at interpolation_factor = 1): the overlay's
-    registry, linear and slerp against the reference's own file, bit for bit."""
-    spec = importlib.util.spec_from_file_location("_ref_pipeline_utils", REF / "src" / "pipelines" / "utils.py")
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    registry, linear and slerp against what the reference's own file computed (tests/golden/pipeline_utils.pt), bit for
+    bit. slerp reduces over the tensor, and ATen's reduction order follows the SIMD width it dispatches to: the fixture
+    records the capability it was written with (AVX512); on a CPU of another capability slerp is held to a few ulp."""
     import src.pipelines.utils as ours
-    g = torch.Generator().manual_seed(3)
-    a, b = torch.randn(4, 8, 8, generator=g), torch.randn(4, 8, 8, generator=g)
+    want = torch.load(golden_dir / "pipeline_utils.pt")
+    a, b = want["a"], want["b"]
+    same_isa = torch.backends.cpu.get_cpu_capability() == want["cpu_capability"]
     for t in (0.0, 0.25, 0.5, 0.9):
-        assert torch.equal(ours.linear(a, b, t), ref.linear(a, b, t))
-        assert torch.equal(ours.slerp(a, b, t), ref.slerp(a, b, t))
-        assert torch.equal(ours.slerp(a, a * 1.0001, t), ref.slerp(a, a * 1.0001, t))  # nearly parallel: the linear branch
+        assert torch.equal(ours.linear(a, b, t), want[f"linear-{t}"])
+        for name, v1 in (("slerp", b), ("slerp_parallel", a * 1.0001)):  # nearly parallel: the linear branch
+            got, ref = ours.slerp(a, v1, t), want[f"{name}-{t}"]
+            assert torch.equal(got, ref) or (not same_isa and torch.allclose(got, ref, rtol=1e-6, atol=1e-7))
     for flag in (True, False):
         ours.set_tensor_interpolation_method(flag)
-        ref.set_tensor_interpolation_method(flag)
-        assert ours.get_tensor_interpolation_method().__name__ == ref.get_tensor_interpolation_method().__name__
+        assert ours.get_tensor_interpolation_method().__name__ == want[f"method-{flag}"]

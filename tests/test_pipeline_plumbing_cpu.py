@@ -5,11 +5,13 @@ backgrounds, joint VAE encode, conditional-half reference pass, context windows,
 with the engine entry points replaced, in this test only, by oracle-backed stand-ins (the product has no CPU path), against
 the golden clip the reference's own pipeline produced (tests/golden/pipeline_cfg1.pt). Every line of host logic between the
 public inputs and the engine calls runs for real; the kernels behind those calls are pinned on the GPU."""
+from types import SimpleNamespace
+
 import numpy as np
 import pytest
 import torch
 
-from test_dropin_cpu import REF, _oracle_engines  # noqa: F401  (same stand-ins as the drop-in proof)
+from oracle.dropin import oracle_engines  # same stand-ins as the drop-in proof
 
 
 class _Event:
@@ -23,8 +25,9 @@ class _Event:
         return 0.0
 
 
-@pytest.mark.parametrize("F_,guidance", [(1, 3.5), (26, 3.5), (26, 1.0)])
-def test_own_sampler_host_logic_on_cpu(monkeypatch, golden_dir, F_, guidance):
+def own_sampler_clip(monkeypatch, golden_dir, F_, guidance):
+    """One clip of this repo's sampler over oracle-backed engines: BASELINE configs[0] (F_ = 1) or the 26-frame,
+    two-window case at 64x64 (then also the same clip from oracle.sample_clip as `ref_out`)."""
     import PIL.Image
     from transformers import CLIPVisionConfig, CLIPVisionModelWithProjection
 
@@ -40,7 +43,7 @@ def test_own_sampler_host_logic_on_cpu(monkeypatch, golden_dir, F_, guidance):
     widths = (128, 256, 512, 512)
     cfg = O.UNetConfig(block_out_channels=widths)
     vcfg = O.VAEConfig(block_out_channels=tuple(g["vae_widths"]) if F_ == 1 else (32, 64, 128, 128))
-    _oracle_engines(monkeypatch, O, cfg, vcfg)
+    oracle_engines(monkeypatch, O, cfg, vcfg)
     monkeypatch.setattr(torch.cuda, "Event", _Event)
 
     def cfg_ddim(pu, pc, latents, guidance, sa_t, s1a_t, sa_p, s1a_p, *, counter=None, frame_stride=0):
@@ -94,8 +97,24 @@ def test_own_sampler_host_logic_on_cpu(monkeypatch, golden_dir, F_, guidance):
         seen, never = [], []
         out = pipe.sample_tensors(host, steps, guidance, callback=lambda i, t, lat: seen.append((i, int(t), tuple(lat.shape))))
         pipe.sample_tensors(host, 1, guidance, callback=lambda *a: never.append(a), callback_steps=2, decode=False)
+    ref_out = None
+    if F_ != 1:
+        with torch.no_grad():
+            emb = clip(pipe._clip_pixels(ref_img)).image_embeds
+            lat0 = torch.randn((1, 4, F_, size // 8, size // 8), generator=torch.manual_seed(42), dtype=torch.float32)
+            W = O.Weights(sds["den"], sds["ref"], sds["pg"], sds["vae"], cfg, vcfg)
+            ref_out = O.sample_clip(W, pil_to_tensor(ref_img, size, size, True),
+                                    pil_to_tensor(poses, size, size, False).permute(1, 0, 2, 3).unsqueeze(0),
+                                    pil_to_tensor(bks, size, size, True), emb, lat0, steps, guidance)
+    return SimpleNamespace(out=out, seen=seen, never=never, ref_out=ref_out, golden=g, size=size, den=den)
+
+
+@pytest.mark.parametrize("F_,guidance", [(1, 3.5), (26, 3.5), (26, 1.0)])
+def test_own_sampler_host_logic_on_cpu(monkeypatch, golden_dir, F_, guidance):
+    r = own_sampler_clip(monkeypatch, golden_dir, F_, guidance)
+    out, seen, never, ref_out, g, size = r.out, r.seen, r.never, r.ref_out, r.golden, r.size
     # the reference's callback sees the shadowed loop variable (pipeline :503-510, :556-561): the index of the last context
-    # batch at every step - pinned on the reference's own file in tests/test_dropin_cpu.py
+    # batch at every step - pinned against the reference's own pipeline file in tests/test_dropin_cpu.py
     nwin = 1 if F_ == 1 else 2
     assert seen == [(nwin - 1, t, (1, 4, F_, size // 8, size // 8)) for t in (999, 499)]
     assert len(never) == (1 if nwin == 1 else 0)  # (nwin - 1) % 2: 0 -> called, 1 -> never
@@ -107,13 +126,6 @@ def test_own_sampler_host_logic_on_cpu(monkeypatch, golden_dir, F_, guidance):
         assert err < 2e-3, err  # the fixture is stored in fp16
         assert float((out["latents"] - g["latents"].float()).norm() / g["latents"].float().norm()) < 2e-3
     else:
-        with torch.no_grad():
-            emb = clip(pipe._clip_pixels(ref_img)).image_embeds
-            lat0 = torch.randn((1, 4, F_, size // 8, size // 8), generator=torch.manual_seed(42), dtype=torch.float32)
-            W = O.Weights(sds["den"], sds["ref"], sds["pg"], sds["vae"], cfg, vcfg)
-            ref_out = O.sample_clip(W, pil_to_tensor(ref_img, size, size, True),
-                                    pil_to_tensor(poses, size, size, False).permute(1, 0, 2, 3).unsqueeze(0),
-                                    pil_to_tensor(bks, size, size, True), emb, lat0, steps, guidance)
         err = float((out["latents"] - ref_out["latents"]).norm() / ref_out["latents"].norm())
         assert err < 1e-4, err  # fp32 both sides: only summation-order noise
         assert float((vid.float() - ref_out["videos"]).norm() / ref_out["videos"].norm()) < 1e-4
