@@ -76,12 +76,6 @@ typedef struct {
   int32_t K1;      /* columns of `a1` (0 if a1 == NULL); w is [N, K + K1] */
   int32_t dtype;
   mimo_epilogue ep;
-  /* optional scratch (device, 16-byte aligned, contents irrelevant, may be shared by all calls of a stream): lets small-M /
-   * long-K problems split the K loop over several CTAs (fp32 partials, summed in a fixed order by a second kernel:
-   * deterministic). NULL = never split. (Disabled by default inside the library: measured slower on B200 at the shapes
-   * of this path - see csrc/gemm_tcgen05.cu.) */
-  void* workspace;
-  int64_t workspace_bytes;
 } mimo_gemm_params;
 int mimo_gemm(const mimo_gemm_params* p, void* stream);
 /* number of value rows (== gate rows) per packed GEGLU tile for a packed width N (N = 2 * out features) */
@@ -105,8 +99,6 @@ typedef struct {
   int32_t n, h, w_, cout;
   int32_t dtype;
   mimo_epilogue ep;
-  void* workspace; /* as in mimo_gemm_params */
-  int64_t workspace_bytes;
 } mimo_conv3x3_params;
 int mimo_conv3x3(const mimo_conv3x3_params* p, void* stream);
 /* Upsample3D (src/models/resnet.py:53-90): nearest x2 (H, W) followed by the 3x3 / pad 1 conv, WITHOUT materialising

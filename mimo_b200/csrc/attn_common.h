@@ -1,5 +1,7 @@
-// Shared declarations of the spatial-attention kernels (attn_spatial.cu: one Q tile per CTA, any head dim up to 192;
-// attn_spatial_pp.cu: two Q tiles per CTA in ping-pong, head dim <= 128).
+// Shared declarations of the spatial-attention kernels. mimo_attn_spatial (attn_spatial.cu) picks one by head dim:
+//   d + 1 <= 64 : attn_spatial_pp2.cu - two Q tiles per CTA in ping-pong, two softmax threads per query row
+//   dp <= 128   : attn_spatial_pp.cu  - two Q tiles per CTA in ping-pong, one softmax thread per query row
+//   otherwise   : attn_spatial.cu     - one Q tile per CTA, head dim up to 192
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -17,16 +19,13 @@ struct AttnArgs {
   const int* bank_index;
   void* out;
   long long ld_out;
-  int variant;        // debug (mimo_debug_attn_variant) bits: 4 = P stores deferred, 8 = no stagger
-  long long* trace;   // debug (mimo_debug_attn_trace): clock64 timeline of CTA (0,0,0), or nullptr
 };
 
 // two Q tiles per CTA (grid.x = ceil(lq / 256)); dp <= 128
 int launch_attn_pp(bool bf16, const CUtensorMap& q, const CUtensorMap& k, const CUtensorMap& v, const CUtensorMap& bk,
                    const CUtensorMap& bv, const AttnArgs& a, int n, cudaStream_t st);
 
-// two softmax threads per query row, row sum by the tensor pipe (attn_spatial_pp2.cu); d + 1 <= 128
-bool attn_pp2_supports(int d);
+// two softmax threads per query row, row sum by the tensor pipe (attn_spatial_pp2.cu); d + 1 <= 64
 int launch_attn_pp2(bool bf16, const CUtensorMap& q, const CUtensorMap& k, const CUtensorMap& v, const CUtensorMap& bk,
                     const CUtensorMap& bv, const AttnArgs& a, int n, cudaStream_t st);
 

@@ -1,4 +1,6 @@
-// Spatial self-attention with the reference-image bank: flash attention on tcgen05.
+// Spatial self-attention with the reference-image bank: flash attention on tcgen05. This file holds the entry point,
+// which picks the kernel by head dim (see attn_common.h), and the single-tile kernel used for d > 128 (the UNet's
+// 16x16 and 8x8 levels: d = 160).
 //
 // One CTA = 128 query rows of one (frame-sample n, head h). The key/value sequence is [self tokens | bank
 // tokens of branch bank_index[n]] (bank skipped when bank_index[n] < 0: the unconditional CFG half attends to
@@ -22,7 +24,6 @@
 namespace mimo {
 
 constexpr int kAttnThreads = 256;
-static int g_attn_variant = 0;  // test hook: 0 = auto, 1 = force the single-tile kernel
 
 template <int NCH, int KVST>
 struct AttnCfg {
@@ -279,7 +280,7 @@ attn_spatial_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
 
 template <int NCH, int KVST, bool kBf16>
 static int launch_attn(const CUtensorMap& q, const CUtensorMap& k, const CUtensorMap& v, const CUtensorMap& bk,
-                       const CUtensorMap& bv, const AttnArgs& a, dim3 grid, cudaStream_t st) {
+                       const CUtensorMap& bv, const AttnArgs& a, int n, cudaStream_t st) {
   using Cfg = AttnCfg<NCH, KVST>;
   auto kern = attn_spatial_kernel<NCH, KVST, kBf16>;
   static bool attr_done = false;
@@ -288,6 +289,7 @@ static int launch_attn(const CUtensorMap& q, const CUtensorMap& k, const CUtenso
     if (e != cudaSuccess) return set_cuda_error("cudaFuncSetAttribute(attn)", e);
     attr_done = true;
   }
+  dim3 grid((a.lq + BQ - 1) / BQ, a.heads, n);
   cudaError_t e = launch_k(kern, grid, dim3(kAttnThreads), Cfg::kSmemBytes, st, q, k, v, bk, bv, a);
   if (e == cudaSuccess) e = cudaGetLastError();
   if (e != cudaSuccess) return set_cuda_error("attn launch", e);
@@ -308,16 +310,6 @@ static int attn_tmap(CUtensorMap* m, int dtype, const void* base, int d, int hea
 
 using namespace mimo;
 
-extern "C" int mimo_debug_attn_variant(int v) {
-  g_attn_variant = v;
-  return 0;
-}
-static long long* g_attn_trace = nullptr;
-extern "C" int mimo_debug_attn_trace(void* buf) {  // >= 5120 int64 of device memory, or NULL
-  g_attn_trace = static_cast<long long*>(buf);
-  return 0;
-}
-
 extern "C" int mimo_attn_spatial(const mimo_attn_params* p, void* stream) {
   if (!p || !p->q || !p->k || !p->v || !p->out) return set_error(MIMO_ERR_ARG, "mimo_attn_spatial: null pointer");
   if (p->n <= 0 || p->lq <= 0 || p->heads <= 0 || p->d <= 0 || (p->d % 8) || p->d > 192 || (p->ld_qkv % 8) ||
@@ -329,8 +321,6 @@ extern "C" int mimo_attn_spatial(const mimo_attn_params* p, void* stream) {
 
   AttnArgs a;
   a.lq = p->lq;
-  a.variant = g_attn_variant;
-  a.trace = g_attn_trace;
   a.lb = has_bank ? p->lb : 0;
   a.heads = p->heads;
   a.d = p->d;
@@ -354,19 +344,13 @@ extern "C" int mimo_attn_spatial(const mimo_attn_params* p, void* stream) {
     tbk = tk;
     tbv = tv;
   }
-  dim3 grid((p->lq + BQ - 1) / BQ, p->heads, p->n);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int nch = (a.dp + 63) / 64;
   const bool bf = p->dtype == MIMO_BF16;
   // d + 1 <= 64 (the 64x64 level, d = 40: MUFU-bound): two softmax threads per row + row sum on the tensor pipe
-  // (attn_spatial_pp2.cu; measured 467 vs 429 TFLOP/s). Variant bit 16 forces it wherever it applies, bit 32 disables it.
-  if (attn_pp2_supports(p->d) && !(g_attn_variant & 32) && g_attn_variant != 1 && ((g_attn_variant & 16) || p->d + 1 <= 64))
-    return launch_attn_pp2(bf, tq, tk, tv, tbk, tbv, a, p->n, st);
-  if (nch <= 2 && g_attn_variant != 1) return launch_attn_pp(bf, tq, tk, tv, tbk, tbv, a, p->n, st);
-  if (nch == 1) return bf ? launch_attn<1, 2, true>(tq, tk, tv, tbk, tbv, a, grid, st)
-                          : launch_attn<1, 2, false>(tq, tk, tv, tbk, tbv, a, grid, st);
-  if (nch == 2) return bf ? launch_attn<2, 2, true>(tq, tk, tv, tbk, tbv, a, grid, st)
-                          : launch_attn<2, 2, false>(tq, tk, tv, tbk, tbv, a, grid, st);
-  return bf ? launch_attn<3, 1, true>(tq, tk, tv, tbk, tbv, a, grid, st)
-            : launch_attn<3, 1, false>(tq, tk, tv, tbk, tbv, a, grid, st);
+  // (attn_spatial_pp2.cu; measured 467 vs 429 TFLOP/s)
+  if (p->d + 1 <= 64) return launch_attn_pp2(bf, tq, tk, tv, tbk, tbv, a, p->n, st);
+  if (a.dp <= 128) return launch_attn_pp(bf, tq, tk, tv, tbk, tbv, a, p->n, st);
+  // d <= 192: three 64-wide chunks, one KV stage
+  return bf ? launch_attn<3, 1, true>(tq, tk, tv, tbk, tbv, a, p->n, st)
+            : launch_attn<3, 1, false>(tq, tk, tv, tbk, tbv, a, p->n, st);
 }

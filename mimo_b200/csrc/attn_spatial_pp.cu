@@ -1,5 +1,5 @@
-// Spatial self-attention with the reference bank, head dim <= 64 (the UNet's 64x64 level: d = 40, 87 % of all
-// attention FLOPs): flash attention with TWO 128-row query tiles per CTA processed in ping-pong.
+// Spatial self-attention with the reference bank, head dims 64 to 128 (CLIP: d = 64; the UNet's 32x32 level: d = 80):
+// flash attention with TWO 128-row query tiles per CTA processed in ping-pong.
 //
 //   warp 0 lane 0 : TMA      - Q tiles A and B once; K/V tiles in rings shared by both query tiles
 //   warp 1 / 3    : MMA      - warp 1 drives query tile A, warp 3 tile B (whole warp + one elected lane, descriptors in
@@ -11,7 +11,7 @@
 //                              waits run under the other group's MUFU work instead of both idling the pipe together
 // A softmax thread pulls its whole 128-key row of S into registers (128 of the 168 the launch bound allows) and
 // releases S_X at once, so Q_X K[j+1]^T runs underneath the exponentials of tile j and
-// the MUFU pipe - the bound of this kernel at d = 40 - never waits for the tensor pipe.
+// the MUFU pipe never waits for the tensor pipe.
 // Softmax: base-2 exponentials (ex2.approx), fp32 running sum, LAZY rescaling — the reference maximum of a row is only
 // moved (and O rescaled in TMEM) when the tile maximum exceeds it by more than 2^8, which keeps P within fp16
 // range and is exact after the final division by the row sum. P goes to shared memory as the 128B-swizzled K-major A
@@ -152,9 +152,6 @@ attn_spatial_pp_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
     const uint32_t pa0 = smem_u32(sP) + x * 2 * kChunkBytes;
     const uint32_t tS = tmem_base + x * 128;
     const uint32_t tO = tmem_base + 256 + x * 128;
-    long long* tr = (a.trace && lane == 0 && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0)
-                        ? a.trace + 4096 + x * 512
-                        : nullptr;
     auto issue_qk = [&](int j) {
       const uint32_t k_addr = smem_u32(sK + (j % ST) * Cfg::kTile);
       if (elect_one()) {
@@ -176,17 +173,12 @@ attn_spatial_pp_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       const int stage = j % ST;
       if (j + 1 < T) {  // S_X(j+1) as soon as the softmax group has S_X(j) in registers
         mbar_wait(&s_free[x], j & 1);
-        if (tr && j < 64) tr[8 * j] = clock64();
         mbar_wait(&k_full[(j + 1) % ST], ((j + 1) / ST) & 1u);
-        if (tr && j < 64) tr[8 * j + 1] = clock64();
         tc_fence_after();
         issue_qk(j + 1);
-        if (tr && j < 64) tr[8 * j + 2] = clock64();
       }
       mbar_wait(&p_full[x], j & 1);
-      if (tr && j < 64) tr[8 * j + 3] = clock64();
       mbar_wait(&v_full[stage], (j / ST) & 1u);
-      if (tr && j < 64) tr[8 * j + 4] = clock64();
       tc_fence_after();
       const uint32_t v_addr = smem_u32(sV + stage * Cfg::kTile);
       if (elect_one()) {
@@ -200,7 +192,6 @@ attn_spatial_pp_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
         tc_commit(&o_done[x]);
       }
       __syncwarp();
-      if (tr && j < 64) tr[8 * j + 5] = clock64();
     }
    }
   } else {
@@ -215,21 +206,14 @@ attn_spatial_pp_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
     const int sw = r & 7;
     const float sc = a.scale_log2;
     float m_ref = 0.f, l = 0.f;
-    long long* tr = (a.trace && lane == 0 && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0)
-                        ? a.trace + (x * 4 + ew) * 512
-                        : nullptr;
-    const bool early = (a.variant & 4) == 0;
-#define MIMO_TR(k) if (tr && j < 64) tr[j * 8 + (k)] = clock64()
     for (int j = 0; j < T; ++j) {
       const bool bank = j >= a.n_self_tiles;
       const int len = bank ? a.lb : a.lq;
       const int row0 = (bank ? j - a.n_self_tiles : j) * BKV;
       int valid = len - row0;
       if (valid > BKV) valid = BKV;
-      MIMO_TR(0);
       mbar_wait(&s_full[x], j & 1);
       tc_fence_after();
-      MIMO_TR(1);
       // ---- the whole row of S -> registers, then hand S_X back to the tensor pipe ----
       uint32_t sv[4][32];
       tmem_ld_x32(tS, sv[0]);
@@ -240,7 +224,6 @@ attn_spatial_pp_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&s_free[x]);
-      MIMO_TR(2);
       // ---- tile maximum (4 independent chains) ----
       float mx0 = -INFINITY, mx1 = -INFINITY, mx2 = -INFINITY, mx3 = -INFINITY;
       if (valid == BKV) {
@@ -277,7 +260,7 @@ attn_spatial_pp_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       // their exponentials (each at half rate), then both in their MUFU-free part - so B is held back once, by
       // the length of A's first exponential phase, and from then on one group's loads / stores / waits hide under
       // the other's exponentials.
-      if (j == 0 && x == 1 && !(a.variant & 8)) mbar_wait(stagger, 0);
+      if (j == 0 && x == 1) mbar_wait(stagger, 0);
       // ---- probabilities (packed in registers) ----
       float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
       const float nm = -m_ref;
@@ -301,32 +284,11 @@ attn_spatial_pp_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
           __syncwarp();
           if (lane == 0) mbar_arrive(stagger);
         }
-        if (early) {
-          if (c == 0 && j > 0) {
-            MIMO_TR(3);
-            mbar_wait(&o_done[x], (j - 1) & 1);
-            tc_fence_after();
-            MIMO_TR(4);
-          }
-          uint8_t* line = prow + (c >> 1) * kChunkBytes;
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            const int piece = (c & 1) * 4 + q;
-            *reinterpret_cast<uint4*>(line + ((piece ^ sw) << 4)) =
-                make_uint4(pk[c * 16 + 4 * q], pk[c * 16 + 4 * q + 1], pk[c * 16 + 4 * q + 2], pk[c * 16 + 4 * q + 3]);
-          }
+        // P_X (and O_X) may only be overwritten once the previous P_X.V has retired
+        if (c == 0 && j > 0) {
+          mbar_wait(&o_done[x], (j - 1) & 1);
+          tc_fence_after();
         }
-      }
-      // P_X (and O_X) may only be overwritten once the previous P_X.V has retired - by now it has, the wait is free
-      if (!early) {
-      if (j > 0) {
-        MIMO_TR(3);
-        mbar_wait(&o_done[x], (j - 1) & 1);
-        tc_fence_after();
-        MIMO_TR(4);
-      }
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
         uint8_t* line = prow + (c >> 1) * kChunkBytes;
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
@@ -335,8 +297,6 @@ attn_spatial_pp_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
               make_uint4(pk[c * 16 + 4 * q], pk[c * 16 + 4 * q + 1], pk[c * 16 + 4 * q + 2], pk[c * 16 + 4 * q + 3]);
         }
       }
-      }
-      MIMO_TR(5);
       l += (s0 + s1) + (s2 + s3);
       // ---- correction of O (rare) ----
       if (rescale) {
@@ -354,7 +314,6 @@ attn_spatial_pp_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_con
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&p_full[x]);
-      MIMO_TR(6);
     }
     // ---- epilogue: O / l -> global ----
     mbar_wait(&o_done[x], (T - 1) & 1);

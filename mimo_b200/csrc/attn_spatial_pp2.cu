@@ -1,5 +1,6 @@
-// Spatial self-attention with the reference bank, head dim <= 112: the ping-pong flash attention of attn_spatial_pp.cu
-// with TWO softmax threads per query row and the row sum computed by the tensor pipe.
+// Spatial self-attention with the reference bank, head dims with d + 1 <= 64 (the UNet's 64x64 level: d = 40): the
+// ping-pong flash attention of attn_spatial_pp.cu with TWO softmax threads per query row and the row sum computed by
+// the tensor pipe.
 //
 // Why: at d = 40 the kernel is bound by the MUFU pipe (16 ex2 / clk / SM). With one thread per row (128 S values in
 // registers, 8 softmax warps) every SM sub-partition hosts two softmax warps whose exponential phases and MUFU-free phases
@@ -275,7 +276,7 @@ attn_spatial_pp2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
           m_ref = mx;
         }
       }
-      if (j == 0 && x == 1 && !(a.variant & 8)) mbar_wait(stagger, 0);
+      if (j == 0 && x == 1) mbar_wait(stagger, 0);
       // P_X (and O_X) may only be overwritten once the previous P_X.V has retired
       if (j > 0) {
         mbar_wait(&o_done[x], (j - 1) & 1);
@@ -383,13 +384,10 @@ static int launch_pp2(const CUtensorMap& q, const CUtensorMap& k, const CUtensor
   return MIMO_OK;
 }
 
-// head dims whose value channels plus the ones column fit the staged tiles: d + 1 <= 64 * NCH and d % 8 == 0
-bool attn_pp2_supports(int d) { return d % 8 == 0 && d + 1 <= 128 && (d + 1 + 15) / 16 * 16 <= 128; }
-
+// the value channels plus the ones column fit one 64-channel chunk: d + 1 <= 64
 int launch_attn_pp2(bool bf16, const CUtensorMap& q, const CUtensorMap& k, const CUtensorMap& v, const CUtensorMap& bk,
                     const CUtensorMap& bv, const AttnArgs& a, int n, cudaStream_t st) {
-  if (a.d + 1 <= 64) return bf16 ? launch_pp2<1, true>(q, k, v, bk, bv, a, n, st) : launch_pp2<1, false>(q, k, v, bk, bv, a, n, st);
-  return bf16 ? launch_pp2<2, true>(q, k, v, bk, bv, a, n, st) : launch_pp2<2, false>(q, k, v, bk, bv, a, n, st);
+  return bf16 ? launch_pp2<1, true>(q, k, v, bk, bv, a, n, st) : launch_pp2<1, false>(q, k, v, bk, bv, a, n, st);
 }
 
 }  // namespace mimo

@@ -51,7 +51,6 @@ struct EpiArgs {
   float scale;
   int act;
   long long* trace;  // debug (mimo_debug_gemm_trace): clock64 timeline of CTA 0, or nullptr
-  float* partial;    // split-K: fp32 accumulators go to partial[split][row][N] instead of the epilogue (else nullptr)
 };
 
 struct ConvGeom {
@@ -64,8 +63,6 @@ struct ConvGeom {
   int kb0, kb1;     // 64-wide K blocks (per tap in conv mode) of source 0 / 1
   int a_bytes;      // bytes one A box deposits in shared memory
   int chunk_bytes;  // bytes one output / residual box moves (TW*TH*TN rows x 64 B)
-  int splits;       // split-K factor (1 = off): tile index = (m_tile * n_tiles + n_tile) * splits + split
-  int kb_split;     // K blocks per split
   int ntaps;        // 9 (3x3) or 4 (one parity class of nearest-x2 upsample + 3x3, see mimo_conv_up2x)
   signed char tdx[9], tdy[9];  // input offset of tap t relative to the output pixel
 };
@@ -114,17 +111,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
   pdl_launch_dependents();
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);  // provably warp-uniform for the compiler
   const int lane = threadIdx.x & 31;
-  const int num_tiles = num_m_tiles * num_n_tiles * g.splits;
-  // tile -> (output tile, K range): with split-K several CTAs share an output tile and each takes kb_split K blocks
-  auto decode = [&](int tile, int& m_tile, int& n_tile, int& split, int& kb_begin, int& kb_cnt) {
-    const int mn = tile / g.splits;
-    split = tile - mn * g.splits;
-    m_tile = mn / num_n_tiles;
-    n_tile = mn - m_tile * num_n_tiles;
-    kb_begin = split * g.kb_split;
-    kb_cnt = num_k_blocks - kb_begin;
-    if (kb_cnt > g.kb_split) kb_cnt = g.kb_split;
-  };
+  const int num_tiles = num_m_tiles * num_n_tiles;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA0);
@@ -177,15 +164,14 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
     uint32_t it = 0, stage = 0, phase = 0;
     const int kb_per_tap = g.kb0 + g.kb1;
     for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-      int m_tile, n_tile, split, kb_begin, kb_cnt;
-      decode(tile, m_tile, n_tile, split, kb_begin, kb_cnt);
+      const int m_tile = tile / num_n_tiles;
+      const int n_tile = tile % num_n_tiles;
       int x0, y0, n0;
       tile_origin(m_tile, x0, y0, n0);
-      // conv: k-block inside the tap, tap index / offsets, tap * ctot (one division per tile, only under split-K)
-      int tap = kb_per_tap > 0 ? kb_begin / kb_per_tap : 0;
-      int rem = kb_begin - tap * kb_per_tap;
-      int dx = g.tdx[tap], dy = g.tdy[tap], tap_k = tap * g.ctot;
-      for (int kbl = 0, kb = kb_begin; kbl < kb_cnt; ++kbl, ++kb, ++it) {
+      // conv: k-block inside the tap, tap index / offsets, tap * ctot
+      int tap = 0, rem = 0;
+      int dx = g.tdx[0], dy = g.tdy[0], tap_k = 0;
+      for (int kb = 0; kb < num_k_blocks; ++kb, ++it) {
         mbar_wait(&empty_bar[stage], phase ^ 1u);
         if (ep.trace && blockIdx.x == 0 && lane == 0 && it < 512) ep.trace[2560 + it] = clock64();
         uint8_t* sa = smem + stage * Cfg::kStageBytes;
@@ -239,9 +225,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
       long long* trm = (ep.trace && blockIdx.x == 0 && lane == 0 && lt < 32) ? ep.trace + 2048 + lt * 16 : nullptr;
       if (trm) trm[0] = clock64();
       const uint32_t d_tmem = tmem_base + acc * BN;
-      int m_tile_, n_tile_, split_, kb_begin_, kb_cnt;
-      decode(tile, m_tile_, n_tile_, split_, kb_begin_, kb_cnt);
-      for (int kb = 0; kb < kb_cnt; ++kb) {
+      for (int kb = 0; kb < num_k_blocks; ++kb) {
         mbar_wait(&full_bar[stage], phase);
         tc_fence_after();
         if (trm && kb < 12) trm[1 + kb] = clock64();
@@ -256,7 +240,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
             umma_ss(d_tmem, da + 2 * k, db + 2 * k, idesc, (kb | k) != 0 ? 1u : 0u);
           }
           tc_commit(&empty_bar[stage]);  // frees the smem stage once these MMAs have read it
-          if (kb == kb_cnt - 1) tc_commit(&tmem_full[acc]);  // accumulator complete -> epilogue
+          if (kb == num_k_blocks - 1) tc_commit(&tmem_full[acc]);  // accumulator complete -> epilogue
         }
         __syncwarp();
         if (++stage == Cfg::kStages) {
@@ -275,7 +259,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
       constexpr int IMAX = grp_count(NCHUNK, 0);
       uint32_t cnt[kEpiGroups] = {};
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        const int m_tile = tile / num_n_tiles;  // (a residual never comes with split-K: splits == 1 here)
+        const int m_tile = tile / num_n_tiles;
         const int n_tile = tile % num_n_tiles;
         int x0, y0, n0;
         tile_origin(m_tile, x0, y0, n0);
@@ -319,8 +303,8 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
     for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++lt) {
       tk = 0;
       GEMM_TR();  // 0: tile start
-      int m_tile, n_tile, split, kb_begin_e, kb_cnt_e;
-      decode(tile, m_tile, n_tile, split, kb_begin_e, kb_cnt_e);
+      const int m_tile = tile / num_n_tiles;
+      const int n_tile = tile % num_n_tiles;
       const uint32_t acc = lt & 1u;
       const uint32_t acc_phase = (lt >> 1) & 1u;
       int x0, y0, n0;
@@ -361,7 +345,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
       const int ce = (warp - 4) * 32 + lane;  // one column per epilogue thread (BN <= 256)
       auto load_consts = [&](int t) -> float {
         float v = 0.f;
-        const int mt = (t / g.splits) / num_n_tiles, nt = (t / g.splits) % num_n_tiles;
+        const int mt = t / num_n_tiles, nt = t % num_n_tiles;
         const int col = nt * BN + ce;
         if (ce < BN && col < N) {
           if (ep.bias) v = C::to_f(static_cast<const T*>(ep.bias)[col]);
@@ -396,27 +380,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
       tc_fence_after();
       GEMM_TR();  // 2: accumulator ready
 
-      if (ep.partial) {
-        // split-K: raw fp32 accumulators of this K range -> partial[split][row][N]; the reduction kernel sums the
-        // splits in a fixed order and applies the whole epilogue (deterministic: no atomics)
-        const int cbase = grp_base(NCHUNK, hsel);
-        const int ccount = grp_count(NCHUNK, hsel);
-        float* prow = ep.partial + (static_cast<long long>(split) * M + row) * N;
-#pragma unroll 1
-        for (int i = 0; i < ccount; ++i) {
-          const int c = cbase + i;
-          uint32_t v[32];
-          tmem_ld_x32(taddr + c * 32, v);
-          tmem_ld_wait();
-          const int col0 = n_tile * BN + c * 32;
-          if (row_ok) {
-#pragma unroll
-            for (int q = 0; q < 8; ++q)
-              if (col0 + q * 4 < N)
-                *reinterpret_cast<uint4*>(prow + col0 + q * 4) = make_uint4(v[q * 4], v[q * 4 + 1], v[q * 4 + 2], v[q * 4 + 3]);
-          }
-        }
-      } else if (ep.act != MIMO_ACT_GEGLU) {
+      if (ep.act != MIMO_ACT_GEGLU) {
         const int cbase = grp_base(NCHUNK, hsel);
         const int ccount = grp_count(NCHUNK, hsel);
         const float scale = ep.scale;
@@ -608,76 +572,6 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-// split-K reduction + the complete epilogue: out = act((sum_s partial[s] * scale + (bias + rowvec) * scale + residual * scale))
-// in the same operation order as the in-kernel epilogue. 8 columns per thread, splits summed in index order.
-template <bool kBf16>
-__global__ void __launch_bounds__(256)
-splitk_reduce_kernel(const float* __restrict__ part, int splits, long long M, int N, const void* __restrict__ bias,
-                     const void* __restrict__ rowvec, long long rpg, long long ld_rowvec,
-                     const void* __restrict__ res, long long ld_res, float scale, int act, void* __restrict__ out,
-                     long long ldo) {
-  using C = Cvt<kBf16>;
-  using T = typename C::T;
-  pdl_launch_dependents();
-  pdl_wait();
-  const int nv = N >> 3;
-  const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
-  if (idx >= M * nv) return;
-  const long long row = idx / nv;
-  const int col = static_cast<int>(idx - row * nv) * 8;
-  float a[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-  for (int s = 0; s < splits; ++s) {
-    const float4* p = reinterpret_cast<const float4*>(part + (static_cast<long long>(s) * M + row) * N + col);
-    const float4 u0 = p[0], u1 = p[1];
-    a[0] += u0.x, a[1] += u0.y, a[2] += u0.z, a[3] += u0.w;
-    a[4] += u1.x, a[5] += u1.y, a[6] += u1.z, a[7] += u1.w;
-  }
-  float cst[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-  auto add_vec = [&](const T* v, float* dst, bool scaled_fma) {
-    const uint4 b = *reinterpret_cast<const uint4*>(v);
-    const uint32_t w[4] = {b.x, b.y, b.z, b.w};
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const float2 t = C::unpack(w[j]);
-      if (scaled_fma) {
-        dst[2 * j] = fmaf(t.x, scale, dst[2 * j]);
-        dst[2 * j + 1] = fmaf(t.y, scale, dst[2 * j + 1]);
-      } else {
-        dst[2 * j] += t.x;
-        dst[2 * j + 1] += t.y;
-      }
-    }
-  };
-  if (bias) add_vec(static_cast<const T*>(bias) + col, cst, false);
-  if (rowvec) add_vec(static_cast<const T*>(rowvec) + (row / rpg) * ld_rowvec + col, cst, false);
-  float f[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) f[j] = fmaf(a[j], scale, cst[j] * scale);
-  if (res) add_vec(static_cast<const T*>(res) + row * ld_res + col, f, true);
-  if (act == MIMO_ACT_SILU) {
-#pragma unroll
-    for (int j = 0; j < 8; ++j) f[j] = silu_f(f[j]);
-  }
-  uint4 o;
-  o.x = C::pack(f[0], f[1]);
-  o.y = C::pack(f[2], f[3]);
-  o.z = C::pack(f[4], f[5]);
-  o.w = C::pack(f[6], f[7]);
-  *reinterpret_cast<uint4*>(static_cast<T*>(out) + row * ldo + col) = o;
-}
-
-// Split-K decision: only when the output tiles would leave more than half of the SMs idle AND every split still gets a
-// long K range (>= 16 K blocks = 1024): the deep, small-M convolutions / FF projections of the 8x8 and 16x16 levels when
-// the clip's frames are spread over several GPUs. Returns the number of splits (1 = off).
-static int pick_splits(long long tiles, int nkb, long long M, int N, int64_t ws_bytes) {
-  if (tiles * 2 > num_sms() || nkb < 32) return 1;
-  long long s = num_sms() / tiles;
-  if (s > nkb / 16) s = nkb / 16;
-  if (s > 16) s = 16;
-  while (s > 1 && s * M * N * 4 > ws_bytes) --s;
-  return s < 2 ? 1 : static_cast<int>(s);
-}
-
 struct Maps {
   CUtensorMap a0, a1, b, out, res;
 };
@@ -764,40 +658,12 @@ static EpiArgs make_epi(const mimo_epilogue& e, int N) {
   a.scale = e.scale;
   a.act = e.act;
   a.trace = g_gemm_trace;
-  a.partial = nullptr;
   return a;
-}
-
-// Split-K is OFF by default: measured on B200 (profiles/r02_splitk_bench.log) the second kernel and the fp32 partial
-// traffic cost more than the better SM fill buys at every shape of the path (e.g. conv 6x8x8 1280->1280: 60 us un-split,
-// 136 us with 9 splits; 16x16 level: +-2 %), and an M-dependent summation order would break the bit-identity of sharded
-// and un-sharded runs. mimo_debug_splitk(1) enables the automatic choice (tests/test_kernels_gpu.py keeps it honest).
-static int g_splitk = 0;
-
-static int launch_reduce(int dtype, const float* part, int splits, long long M, int N, const mimo_epilogue& e, void* out,
-                         long long ldo, cudaStream_t st) {
-  const long long total = M * (N / 8);
-  const unsigned blocks = div_up(total, 256);
-  const long long rpg = e.rows_per_group > 0 ? e.rows_per_group : 1;
-  const long long ldr = e.ld_rowvec > 0 ? e.ld_rowvec : N;
-  cudaError_t err = dtype == MIMO_BF16
-                        ? launch_k(splitk_reduce_kernel<true>, dim3(blocks), dim3(256), 0, st, part, splits, M, N, e.bias,
-                                   e.rowvec, rpg, ldr, e.residual, static_cast<long long>(e.ld_res), e.scale, e.act, out, ldo)
-                        : launch_k(splitk_reduce_kernel<false>, dim3(blocks), dim3(256), 0, st, part, splits, M, N, e.bias,
-                                   e.rowvec, rpg, ldr, e.residual, static_cast<long long>(e.ld_res), e.scale, e.act, out, ldo);
-  if (err == cudaSuccess) err = cudaGetLastError();
-  if (err != cudaSuccess) return set_cuda_error("split-K reduce launch", err);
-  return MIMO_OK;
 }
 
 }  // namespace mimo
 
 using namespace mimo;
-
-extern "C" int mimo_debug_splitk(int mode) {
-  g_splitk = mode;
-  return 0;
-}
 
 extern "C" int mimo_debug_force_bn(int bn) {
   g_force_bn = bn;
@@ -826,16 +692,10 @@ extern "C" int mimo_gemm(const mimo_gemm_params* p, void* stream) {
   const int kb0 = (p->K + BK - 1) / BK;
   const int kb1 = (K1 + BK - 1) / BK;
   const int nkb = kb0 + kb1;
-  int bn = pick_bn(p->N, geglu, mt);
-  int splits = 1;
-  if (!geglu && g_splitk && p->workspace && !g_force_bn) {
-    const int bn_wide = pick_bn(p->N, false, 1 << 20);  // the tile width a large problem would get
-    splits = pick_splits(static_cast<long long>(mt) * ((p->N + bn_wide - 1) / bn_wide), nkb, p->M, p->N, p->workspace_bytes);
-    if (splits > 1) bn = bn_wide;
-  }
+  const int bn = pick_bn(p->N, geglu, mt);
   if (geglu && (p->N % bn)) return set_error(MIMO_ERR_ARG, "mimo_gemm: GEGLU needs N % tile == 0");
   const int nt = (p->N + bn - 1) / bn;
-  const bool res = p->ep.residual != nullptr && !geglu && splits == 1;
+  const bool res = p->ep.residual != nullptr && !geglu;
 
   Maps m;
   const uint64_t adim[2] = {static_cast<uint64_t>(p->K), static_cast<uint64_t>(p->M)};
@@ -869,20 +729,10 @@ extern "C" int mimo_gemm(const mimo_gemm_params* p, void* stream) {
   g.kb1 = kb1;
   g.c0 = p->K;
   g.chunk_bytes = kChunk;
-  g.splits = splits;
-  g.kb_split = (nkb + splits - 1) / splits;
-  EpiArgs ep = make_epi(p->ep, p->N);
+  const EpiArgs ep = make_epi(p->ep, p->N);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (splits > 1) {
-    ep.bias = ep.rowvec = nullptr;
-    ep.act = MIMO_ACT_NONE;
-    ep.scale = 1.0f;
-    ep.partial = static_cast<float*>(p->workspace);
-  }
-  const int rc = p->dtype == MIMO_BF16 ? launch_bn<true>(bn, res, m, p->M, p->N, mt, nt, nkb, g, ep, st)
-                                       : launch_bn<false>(bn, res, m, p->M, p->N, mt, nt, nkb, g, ep, st);
-  if (rc || splits == 1) return rc;
-  return launch_reduce(p->dtype, ep.partial, splits, p->M, p->N, p->ep, p->out, p->ldo, st);
+  return p->dtype == MIMO_BF16 ? launch_bn<true>(bn, res, m, p->M, p->N, mt, nt, nkb, g, ep, st)
+                               : launch_bn<false>(bn, res, m, p->M, p->N, mt, nt, nkb, g, ep, st);
 }
 
 // One implicit-GEMM convolution launch: `ntaps` taps at offsets (tdx, tdy) over the [n, h, w, c] input(s); the output
@@ -922,19 +772,9 @@ static int conv_launch(const mimo_conv3x3_params* p, const void* w, int ntaps, c
   const int nkb = ntaps * (g.kb0 + g.kb1);
   const long long Mrows = static_cast<long long>(p->n) * p->h * p->w_;
   if (Mrows > 0x7fffffffLL) return set_error(MIMO_ERR_ARG, "mimo_conv: too many pixels");
-  int bn = pick_bn(p->cout, false, mt);
-  int splits = 1;
-  // split-K needs the dense NHWC output (row = pixel index): not for the strided parity classes of mimo_conv_up2x
-  if (g_splitk && p->workspace && !g_force_bn && sx == 1 && sy == 1 && p->ldo == p->cout) {
-    const int bn_wide = pick_bn(p->cout, false, 1 << 20);
-    splits = pick_splits(static_cast<long long>(mt) * ((p->cout + bn_wide - 1) / bn_wide), nkb, Mrows, p->cout,
-                         p->workspace_bytes);
-    if (splits > 1) bn = bn_wide;
-  }
-  g.splits = splits;
-  g.kb_split = (nkb + splits - 1) / splits;
+  const int bn = pick_bn(p->cout, false, mt);
   const int nt = (p->cout + bn - 1) / bn;
-  const bool res = p->ep.residual != nullptr && splits == 1;
+  const bool res = p->ep.residual != nullptr;
 
   Maps m;
   auto nhwc_map = [&](CUtensorMap* tm, const void* base, int c, long long pitch, uint32_t box_c, int swz, int px,
@@ -963,19 +803,10 @@ static int conv_launch(const mimo_conv3x3_params* p, const void* w, int ntaps, c
   if (res)
     if (int rc = nhwc_map(&m.res, p->ep.residual, p->cout, p->ep.ld_res, 32, 64, 1, 1, p->w_, p->h)) return rc;
 
-  EpiArgs ep = make_epi(p->ep, p->cout);
+  const EpiArgs ep = make_epi(p->ep, p->cout);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (splits > 1) {
-    ep.bias = ep.rowvec = nullptr;
-    ep.act = MIMO_ACT_NONE;
-    ep.scale = 1.0f;
-    ep.partial = static_cast<float*>(p->workspace);
-  }
-  const int rc = p->dtype == MIMO_BF16
-                     ? launch_bn<true>(bn, res, m, static_cast<int>(Mrows), p->cout, mt, nt, nkb, g, ep, st)
-                     : launch_bn<false>(bn, res, m, static_cast<int>(Mrows), p->cout, mt, nt, nkb, g, ep, st);
-  if (rc || splits == 1) return rc;
-  return launch_reduce(p->dtype, ep.partial, splits, Mrows, p->cout, p->ep, out, p->ldo, st);
+  return p->dtype == MIMO_BF16 ? launch_bn<true>(bn, res, m, static_cast<int>(Mrows), p->cout, mt, nt, nkb, g, ep, st)
+                               : launch_bn<false>(bn, res, m, static_cast<int>(Mrows), p->cout, mt, nt, nkb, g, ep, st);
 }
 
 static int conv_check(const mimo_conv3x3_params* p, const char* who) {

@@ -42,7 +42,6 @@ class GemmParams(C.Structure):
         ("M", C.c_int32), ("N", C.c_int32), ("K", C.c_int32), ("K1", C.c_int32),
         ("dtype", C.c_int32),
         ("ep", Epilogue),
-        ("workspace", C.c_void_p), ("workspace_bytes", C.c_int64),
     ]
 
 
@@ -55,7 +54,6 @@ class Conv3x3Params(C.Structure):
         ("n", C.c_int32), ("h", C.c_int32), ("w_", C.c_int32), ("cout", C.c_int32),
         ("dtype", C.c_int32),
         ("ep", Epilogue),
-        ("workspace", C.c_void_p), ("workspace_bytes", C.c_int64),
     ]
 
 
@@ -145,8 +143,7 @@ SYMBOLS = {
     "mimo_cfg_ddim_step": (C.c_int, [_VP, _VP, _VP, _I64, _VP, _I64, _F, _F, _F, _F, _F, _I32, _VP]),
 }
 # test hook, not part of the public header
-_DEBUG_SYMBOLS = {"mimo_debug_pdl": (C.c_int, [C.c_int]), "mimo_debug_splitk": (C.c_int, [C.c_int]), "mimo_debug_force_bn": (C.c_int, [C.c_int]), "mimo_debug_attn_variant": (C.c_int, [C.c_int]),
-                  "mimo_debug_attn_trace": (C.c_int, [C.c_void_p]),
+_DEBUG_SYMBOLS = {"mimo_debug_pdl": (C.c_int, [C.c_int]), "mimo_debug_force_bn": (C.c_int, [C.c_int]),
                   "mimo_debug_gemm_trace": (C.c_int, [C.c_void_p])}
 
 _lib = None

@@ -73,20 +73,6 @@ def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
     return t.data_ptr()
 
 
-_WORKSPACE: dict = {}
-WORKSPACE_BYTES = 96 << 20
-
-
-def _workspace(device: torch.device) -> torch.Tensor:
-    """One persistent split-K scratch buffer per device (stable address: captured CUDA graphs keep pointing at it)."""
-    key = (device.type, device.index)
-    ws = _WORKSPACE.get(key)
-    if ws is None:
-        ws = torch.empty(WORKSPACE_BYTES, dtype=torch.uint8, device=device)
-        _WORKSPACE[key] = ws
-    return ws
-
-
 def _epilogue(bias=None, rowvec=None, rows_per_group=1, residual=None, scale=1.0, act=L.ACT_NONE) -> L.Epilogue:
     ep = L.Epilogue()
     ep.bias = _ptr(bias)
@@ -120,8 +106,6 @@ def gemm(a: torch.Tensor, w: torch.Tensor, out: Optional[torch.Tensor] = None, *
     p.M, p.N, p.K = M, N, K
     p.dtype = _dt(a)
     p.ep = _epilogue(bias, rowvec, rows_per_group, residual, scale, act)
-    ws = _workspace(a.device)
-    p.workspace, p.workspace_bytes = ws.data_ptr(), ws.numel()
     kt = K + K1
     with _Call("gemm", 1, 2.0 * M * N * kt, 2.0 * (M * kt + N * kt + M * n_out + (M * N if residual is not None else 0))):
         L.check(L.load().mimo_gemm(C.byref(p), _stream()), "mimo_gemm")
@@ -147,8 +131,6 @@ def conv3x3(x0: torch.Tensor, w: torch.Tensor, n: int, h: int, wd: int, out: Opt
     p.n, p.h, p.w_, p.cout = n, h, wd, cout
     p.dtype = _dt(x0)
     p.ep = _epilogue(bias, rowvec, rows_per_group or h * wd, residual, scale, act)
-    ws = _workspace(x0.device)
-    p.workspace, p.workspace_bytes = ws.data_ptr(), ws.numel()
     M, cin = n * h * wd, c0 + c1
     with _Call("conv3x3", 1, 2.0 * M * cout * 9 * cin,
                2.0 * (M * cin + 9 * cin * cout + M * cout + (M * cout if residual is not None else 0))):
